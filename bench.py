@@ -2,7 +2,7 @@
 """bench.py -- 48 kHz frames/sec of the PercepNet enhancement hot path (rnnoise_process_frame) on B200.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference]
-                  [--streams S] [--frames F] [--nn fp32|tensor]
+                  [--streams S] [--frames F] [--nn fp32|tensor] [--dump-outputs DIR]
 
 One "step" = one pnb_process call: S concurrent streams x F hops of 480 samples per GPU.
 Default workload = BASELINE.json config 3/4: 16 384 streams per GPU (weak scaling: 131 072 on 8 GPUs),
@@ -38,6 +38,25 @@ sys.path.insert(0, ROOT)
 FRAME = 480
 FLOP_PER_FRAME = 15_896_576       # network MAC*2 per hop (SURVEY.md 8d, BASELINE.md 3)
 BYTES_PER_FRAME = 3_840           # 480 f32 in + 480 f32 out
+DUMP_BYTES = 64_000_000           # --dump-outputs writes at most this much
+
+
+def dump_rows(n_rows, row_bytes):
+    """Row indices of an output that --dump-outputs writes: all rows when they fit DUMP_BYTES, else a fixed seeded
+    sample (sorted), the same for the same arguments in every run."""
+    k = max(1, min(n_rows, DUMP_BYTES // row_bytes))
+    if k == n_rows:
+        return np.arange(n_rows)
+    return np.sort(np.random.RandomState(0).choice(n_rows, k, replace=False))
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes {name: float32 or float64 host array} as out_dir/<name>.npy."""
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_BYTES
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), name
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def measured_peaks():
@@ -270,6 +289,10 @@ def run_traindata(args):
         step(W + i)
     ev1.record(stream)
     torch.cuda.synchronize()
+    if args.dump_outputs:                                              # the records of the last timed step
+        rec = d_rec[(W + K - 1) % n_buf]
+        rows = torch.from_numpy(dump_rows(N, F * api.RECORD * 4)).to(device)
+        dump_outputs(args.dump_outputs, {"records": rec[rows].cpu().numpy()})
     launches = eng.launches - launches0
     ms = ev0.elapsed_time(ev1)
     clocks = sampler.stop()
@@ -381,6 +404,9 @@ def run_xcorr(args):
     clocks = sampler.stop()
     value = S * K / (ms * 1e-3)
     periods = d_T.cpu().numpy()
+    if args.dump_outputs:                                              # every step writes the same three arrays
+        dump_outputs(args.dump_outputs, {"period": periods.astype(np.float64), "corr": d_corr.cpu().numpy(),
+                                         "gain": d_gain.cpu().numpy()})
     # end to end: pitch buffers in pinned host memory -> periods / gains in host memory (blocking public call)
     h = [b.cpu().pin_memory() for b in bufs]
     hT, hl = torch.empty(S, dtype=torch.int32).pin_memory(), torch.empty(S, dtype=torch.int32).pin_memory()
@@ -489,6 +515,10 @@ def main():
     ap.add_argument("--plain-calls", action="store_true", help="time pnb_process_device_* (joined into the stream after every "
                     "call) instead of pnb_submit_device_* + pnb_flush")
     ap.add_argument("--no-int16-run", action="store_true", help="skip the second timed run at int16 amplitude scale")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed as "
+                    "DIR/<name>.npy: enhance = out [rows, F*480] float32, the enhanced PCM of a fixed sample of the "
+                    "streams (rank 0's); traindata = records [rows, F, 138] float32, likewise sampled; xcorr = period "
+                    "(float64), corr, gain [units] float32.  At most 64 MB; the inputs are the same in every run")
     args = ap.parse_args()
     if not args.frames:
         args.frames = 100 if args.path == "enhance" else 8
@@ -571,6 +601,10 @@ def main():
     eng.flush(stream.cuda_stream)
     ev1.record(stream)
     barrier()
+    if args.dump_outputs and rank == 0:                     # this rank's enhanced PCM of the last timed step
+        out = outs[(W + K - 1) % n_buf]
+        rows = torch.from_numpy(dump_rows(S, F * FRAME * 4)).to(device)
+        dump_outputs(args.dump_outputs, {"out": out[rows].cpu().numpy()})
     launches = (eng.launches - launches0) * world           # kernels launched inside the timed region (library counter; every rank issues the same schedule)
     ms = ev0.elapsed_time(ev1)
     clocks = sampler.stop() if rank == 0 else None

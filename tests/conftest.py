@@ -8,7 +8,6 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-REFERENCE_TREE = "/root/reference"
 
 
 def pytest_configure(config):
@@ -20,16 +19,6 @@ def oracle():
     from oracle import ffi
     ffi.build()
     return ffi.Oracle()
-
-
-@pytest.fixture(scope="session")
-def reference():
-    """The compiled, unmodified reference (oracle/_ref); absent where /root/reference never existed."""
-    from oracle import ffi
-    ffi.build()
-    if not ffi.Reference.available():
-        pytest.skip("oracle/_ref/libpercepnet_ref.so not built (no /root/reference in this container)")
-    return ffi.Reference()
 
 
 @pytest.fixture(scope="session")

@@ -1,61 +1,18 @@
-"""percepnet_b200.weights.pack_state_dict against the reference's real exporter (dump_percepnet.py): the
-exporter's own monkey-patched `dump_data` methods are run on torch modules carrying our synthetic weights, the
-emitted C arrays are parsed back and must equal our packed arrays exactly.  Needs /root/reference (build
-container only); CPU."""
-import io
-import os
-import re
-import sys
-import types
-
-import numpy as np
-import pytest
-
-from conftest import REFERENCE_TREE
-
-pytestmark = pytest.mark.skipif(not os.path.exists(REFERENCE_TREE), reason="needs /root/reference")
-
-
-def _import_exporter():
-    for m in ("h5py", "tensorboardX", "matplotlib", "matplotlib.pyplot"):
-        sys.modules.setdefault(m, types.ModuleType(m))
-    sys.modules["tensorboardX"].SummaryWriter = object
-    sys.modules["matplotlib"].pyplot = sys.modules["matplotlib.pyplot"]
-    sys.modules["matplotlib.pyplot"].switch_backend = lambda *a, **k: None
-    if REFERENCE_TREE not in sys.path:
-        sys.path.insert(0, REFERENCE_TREE)
-    import dump_percepnet  # noqa: F401  (patches Linear/Conv1d/GRU/Sequential with dump_data)
-    import rnn_train
-    return rnn_train
-
-
-def _arrays(txt):
-    out = {}
-    for m in re.finditer(r"static const float (\w+)\[(\d+)\] = \{([^}]*)\}", txt):
-        out[m.group(1)] = np.array([np.float32(v) for v in m.group(3).replace("\n", " ").split(",") if v.strip()],
-                                   dtype=np.float32)
-        assert out[m.group(1)].size == int(m.group(2))
-    return out
+"""percepnet_b200.weights.pack_state_dict against the reference's real exporter (dump_percepnet.py): the exporter's
+own monkey-patched `dump_data` methods, run on the reference's PercepNet module carrying synth_state_dict(3), emitted
+C arrays whose digests tests/golden/make_golden.py stored in tests/golden/reference_digests.json, with the module's
+state_dict shapes and layer order.  Our packed arrays must equal the emitted ones exactly.  CPU."""
+from util import digest, reference_digests
 
 
 def test_pack_matches_reference_exporter():
-    import torch
     from percepnet_b200.weights import LAYERS, pack_state_dict, synth_state_dict
-    rnn_train = _import_exporter()
+    gold = reference_digests()["exporter"]
     sd = synth_state_dict(3)
-    net = rnn_train.PercepNet()
-    assert set(net.state_dict().keys()) == set(sd.keys())                 # names of rnn_train.py:111-121
-    for k, v in net.state_dict().items():
-        assert tuple(v.shape) == sd[k].shape, k
-    net.load_state_dict({k: torch.from_numpy(v) for k, v in sd.items()})
+    assert {k: list(v.shape) for k, v in sd.items()} == gold["state_dict_shapes"]   # names of rnn_train.py:111-121
     packed = pack_state_dict(sd)
-    # the big 512x512 GRUs share code with gru_rb; dump the cheap layers and one big GRU
-    for name, module in net.named_children():
-        if name in ("gru2", "gru3", "gru_gb", "conv2"):
-            continue
-        f = io.StringIO()
-        module.dump_data(f, name)
-        arrs = _arrays(f.getvalue())
-        for key, got in arrs.items():
-            assert np.array_equal(got, packed.arrays[key].ravel()), key
-    assert [l[0] for l in LAYERS] == [n for n, _ in net.named_children()]   # RNNModel field order
+    # the big 512x512 GRUs share code with gru_rb: the cheap layers and one big GRU were dumped
+    assert gold["arrays"]
+    for key, want in gold["arrays"].items():
+        assert digest(packed.arrays[key].ravel()) == want, key
+    assert [l[0] for l in LAYERS] == gold["layers"]                                   # RNNModel field order
